@@ -2,7 +2,7 @@
 """bench.py -- forward+backward Mpixels/s of the differentiable Gaussian rasterizer on BASELINE config 3
 (1M synthetic "bicycle-shaped" Gaussians, SH degree 3, 1600x1200), the metric BASELINE.json names.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c3] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one camera: GaussianRasterizer.forward (preprocess + tile-count
 difference array -> R to the host -> depth order -> scan -> ranges -> two radix passes over tile ids (the first
@@ -23,8 +23,14 @@ protocol).  The 8 ring cameras of the config are cycled step by step.
   --impl reference : the reference's OWN CUDA path (oracle/_ref/libdgr_ref.so = its unmodified .cu files
            compiled for sm_100a) on the same workload; if that library is absent, the CPU oracle port.
 
-  timing : every number is the MEDIAN of 5 back-to-back regions of K steps (each bracketed by barrier + synchronize);
-           the five region times are reported under "timing".
+  timing : the K timed steps run back to back (a barrier + synchronize on each side); CUDA events on the stream split
+           them into 5 regions of about K/5 steps, every number is the MEDIAN of the regions' times per step, and the
+           region times are reported under "timing".
+  --dump-outputs DIR : after the timed steps, what the last timed step returned to its caller is written as
+           DIR/<name>.npy (float32, float64 for the loss): the image and depth in full, and for the per-Gaussian arrays
+           (radii and the gradients of all inputs) the rows of a fixed seeded sample of at most 65536 Gaussians, listed
+           in gaussian_index.npy. The inputs depend only on the arguments, so two builds can be compared output by
+           output.
   N > 1 also runs BASELINE config 4 (5M Gaussians, 1920x1080) through the Gaussian-sharded rasterizer over all N
            GPUs (strong scaling) and reports it under "sharded_c4": ms/step, Mpixels/s, ratio to the plain rasterizer
            on one GPU measured in the same run, bit-comparison of the 8 frames, per-phase times, exchange bytes.
@@ -268,9 +274,18 @@ class OursRunner:
             wl.join_host_inputs()
         loss = (color * G).sum()
         loss.backward()
+        self.last_out = (color, depth, radii, loss)
         if host:
             return wl.read_back(loss)
         return loss
+
+    def outputs(self):
+        """What the last step handed back to its caller: image, depth, radii, loss and the input gradients."""
+        color, depth, radii, loss = self.last_out
+        L = self.leaf
+        return dict(color=color, depth=depth, radii=radii, loss=loss, grad_means3D=L["means3D"].grad,
+                    grad_means2D=self.means2D.grad, grad_opacities=L["opacities"].grad, grad_shs=L["shs"].grad,
+                    grad_scales=L["scales"].grad, grad_rotations=L["rotations"].grad)
 
     def describe(self):
         from gaussianeditor_b200.rasterizer import _RasterizeGaussians, forward_state_views
@@ -314,15 +329,44 @@ class ReferenceCudaRunner:
         # autograd of loss = (color*G).sum() hands dL/dcolor = G to the rasterizer's backward
         self.g = self.R.backward(dL_dcolor=G, radii=radii, R=R, **common)
         self.last = (radii, R)
+        self.last_out = (color, depth, loss)
         if host:
             return wl.read_back(loss)
         return loss
+
+    def outputs(self):
+        color, depth, loss = self.last_out
+        g = self.g
+        return dict(color=color, depth=depth, radii=self.last[0], loss=loss, grad_means3D=g["dL_dmeans3D"],
+                    grad_means2D=g["dL_dmeans2D"], grad_opacities=g["dL_dopacity"], grad_shs=g["dL_dsh"],
+                    grad_scales=g["dL_dscales"], grad_rotations=g["dL_drotations"])
 
     def describe(self):
         radii, R = self.last
         V = int((radii > 0).sum())
         ntile = ((self.wl.W + 15) // 16) * ((self.wl.H + 15) // 16)
         return dict(P=self.wl.P, V=V, R=int(R), R_per_V=R / max(V, 1), R_per_tile=R / ntile, Ntile=ntile)
+
+
+DUMP_ROWS = 65536
+
+
+def dump_outputs(outs, P, out_dir):
+    """Writes the arrays of `outs` as out_dir/<name>.npy: per-Gaussian arrays (first axis P) on a fixed seeded sample
+    of DUMP_ROWS Gaussians (gaussian_index.npy), the rest in full; float32, the loss in float64. Returns bytes written."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.arange(P) if P <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(P, DUMP_ROWS, replace=False))
+    arrays = {"gaussian_index": idx.astype(np.float64)}
+    for name, t in outs.items():
+        a = t.detach().cpu().numpy()
+        if name != "loss" and a.ndim and a.shape[0] == P:
+            a = a[idx]
+        arrays[name] = a.astype(np.float64 if name == "loss" else np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"--dump-outputs would write {total} bytes"
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return total
 
 
 def cpu_oracle_time(name, P=None, threads=None, budget_s=12.0, max_steps=8):
@@ -551,6 +595,8 @@ def main():
     ap.add_argument("--option", action="append", default=[], help="library tuning option k=v (A/B measurements only)")
     ap.add_argument("--no-sharded", action="store_true", help="skip the config-4 Gaussian-sharded leg at --gpus N > 1")
     ap.add_argument("--sharded-points", type=int, default=None, help="override config 4's Gaussian count (debug only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -577,7 +623,11 @@ def main():
               "l2": "inputs (236 MB params + 192 MB SH grads) exceed the 126 MB L2; no explicit flush",
               "parallelism": f"replicas x{world} (one camera stream per GPU, no data-path collective)"}
 
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
     if use_cpu_port:
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs needs the GPU path (the CPU oracle port is not the timed path)")
         # reference arm without the compiled reference: the CPU oracle port, rank 0 only
         if rank != 0:
             return
@@ -611,46 +661,44 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed_once(n, host):
-        barrier()
-        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        a.record()
-        pending, losses = None, []
-        for i in range(n):
-            cur = runner.step(i + rank * 3, host=host)
-            if host:  # consume step i-1's loss on the host while step i runs on the GPU
-                if pending is not None:
-                    losses.append(pending.wait())
-                pending = cur
-        if pending is not None:
-            losses.append(pending.wait())
-            assert len(losses) == n and all(np.isfinite(losses))
-        b.record()
-        barrier()
-        ms = a.elapsed_time(b)
-        if dist is not None:
-            t = torch.tensor([ms], device=dev)
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-            ms = float(t[0])
-        return ms
-
     REPEATS = 5
 
     def timed(n, host):
-        """The K-step timed region (barrier + synchronize on both sides, CUDA events, max over ranks) is measured
-        REPEATS times back to back and the MEDIAN region is reported: K = 20 steps last 28 ms, so one host hiccup
-        (GC, a page fault, a neighbour rank's launch burst) in a single region used to move the number by 10-20 %.
-        Python's cyclic GC is paused inside the regions for the same reason (it runs between them)."""
+        """The n timed steps run back to back between a barrier + synchronize on each side; CUDA events recorded on
+        the stream split them into REPEATS regions of about n / REPEATS steps, and the MEDIAN time per step over the
+        regions (max over ranks) is reported, as the time of n steps: one host hiccup (GC, a page fault, a neighbour
+        rank's launch burst) in a single region of 20 steps used to move the number by 10-20 %. Python's cyclic GC is
+        paused during the steps for the same reason."""
         import gc
-        runs = []
-        for _ in range(REPEATS):
-            gc.collect()
-            gc.disable()
-            try:
-                runs.append(timed_once(n, host))
-            finally:
-                gc.enable()
-        return statistics.median(runs), runs
+        sizes = [n // REPEATS + (1 if r < n % REPEATS else 0) for r in range(min(REPEATS, n))]
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(len(sizes) + 1)]
+        inner_ends = {int(e) - 1: r + 1 for r, e in enumerate(np.cumsum(sizes)[:-1])}   # last step of a region -> event
+        gc.collect()
+        gc.disable()
+        try:
+            barrier()
+            ev[0].record()
+            pending, losses = None, []
+            for i in range(n):
+                cur = runner.step(i + rank * 3, host=host)
+                if host:  # consume step i-1's loss on the host while step i runs on the GPU
+                    if pending is not None:
+                        losses.append(pending.wait())
+                    pending = cur
+                if i in inner_ends:
+                    ev[inner_ends[i]].record()
+            if pending is not None:
+                losses.append(pending.wait())
+                assert len(losses) == n and all(np.isfinite(losses))
+            ev[-1].record()
+            barrier()
+        finally:
+            gc.enable()
+        runs = torch.tensor([ev[r].elapsed_time(ev[r + 1]) for r in range(len(sizes))], device=dev)
+        if dist is not None:
+            dist.all_reduce(runs, op=dist.ReduceOp.MAX)
+        runs = runs.tolist()
+        return statistics.median(ms / k for ms, k in zip(runs, sizes)) * n, runs
 
     for i in range(max(args.warmup, 3)):
         runner.step(i + rank * 3)
@@ -660,6 +708,7 @@ def main():
     ms, ms_runs = timed(args.steps, host=False)
     clocks = sampler.stop()
     launches = (_lib.launch_count() - launches0) if args.impl == "ours" else None
+    dumped = dump_outputs(runner.outputs(), wl.P, args.dump_outputs) if args.dump_outputs and rank == 0 else None
     for i in range(3):
         runner.step(i, host=True).wait()
     ms_e2e, ms_e2e_runs = timed(args.steps, host=True)
@@ -681,16 +730,19 @@ def main():
             "warmup": max(args.warmup, 3), "ms_per_step": ms / args.steps, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "impl": args.impl,
             "config": config, "clocks": clocks,
-            "timing": {"protocol": f"median of {REPEATS} back-to-back regions of {args.steps} steps each (every region "
-                                   "bracketed by barrier + synchronize, CUDA events, max over ranks)",
+            "timing": {"protocol": f"{args.steps} steps back to back (barrier + synchronize on each side), split by "
+                                   f"CUDA events into {min(REPEATS, args.steps)} regions; median time per step over "
+                                   "the regions, max over ranks",
                        "region_ms": [round(x, 4) for x in ms_runs], "e2e_region_ms": [round(x, 4) for x in ms_e2e_runs]},
             "e2e": {"value": e2e, "unit": "Mpixels/s", "ms_per_step": ms_e2e / args.steps,
                     "h2d_bytes_per_step": 3 * npix * 4 + 36 * 4, "d2h_bytes_per_step": 4,
                     "h2d_GBps_measured": round(h2d_gbps, 1)},
             "workload": desc}
+    if dumped is not None:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "bytes": dumped}
 
     if args.impl == "ours":
-        line["gpu_launches"] = int(launches) // REPEATS   # per timed region of `steps` steps
+        line["gpu_launches"] = int(launches)   # over the `steps` timed steps
         # per-stage CUDA-event timing (separate pass so the headline is not perturbed)
         _lib.set_option("profile", 1)
         _lib.profile_read()
