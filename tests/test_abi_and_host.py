@@ -11,6 +11,7 @@ import torch
 
 from gaussianeditor_b200 import _lib, synth
 from gaussianeditor_b200.rasterizer import GaussianRasterizationSettings, GaussianRasterizer
+from util import OPTION_DEFAULTS, get_option, kernel_options
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -58,7 +59,21 @@ def test_sizing_and_validation_without_gpu_semantics():
     assert rc == -1 and b"scale/rotation pair or precomputed 3D covariance" in lib.gsr_last_error()
     # unknown option
     assert lib.gsr_set_option(b"no_such_option", 1) == -1
-    assert lib.gsr_set_option(b"render_fwd_variant", 2) == 0 and lib.gsr_get_option(b"render_fwd_variant") == 2
+    with kernel_options(render_fwd_variant=2):
+        assert lib.gsr_get_option(b"render_fwd_variant") == 2
+
+
+def test_option_defaults_match_the_compiled_ones():
+    """tests/util.OPTION_DEFAULTS (what kernel_options() and the shape/variant tests treat as "the default") is the
+    Options struct of csrc/common.cuh, and kernel_options() restores what it changed."""
+    text = open(os.path.join(ROOT, "gaussianeditor_b200", "csrc", "common.cuh")).read()
+    body = re.search(r"struct Options \{(.*?)\};", text, re.S).group(1)
+    compiled = {k: int(v) for k, v in re.findall(r"int (\w+) = (-?\d+);", body)}
+    assert compiled == OPTION_DEFAULTS
+    before = {k: get_option(k) for k in compiled}
+    with kernel_options(render_bwd_variant=3, tile_key_bits=32):
+        assert get_option("render_bwd_variant") == 3 and get_option("tile_key_bits") == 32
+    assert {k: get_option(k) for k in compiled} == before
 
 
 def _settings(device):

@@ -297,3 +297,27 @@ def test_precomputed_colour_and_covariance_paths_of_the_oracle():
     g2 = pc.backward(2.0 * G)
     assert np.allclose(g2["dcolor"], 2.0 * g["dcolor"], rtol=0, atol=0)
     base.close(); pc.close(); cv.close()
+
+
+@pytest.mark.parametrize("W,H,scene", [(333, 201, "c3"), (4160, 48, "c3"), (7, 5, "c3"), (333, 201, "adversarial")])
+def test_binning_restatement_equals_the_oracle(W, H, scene):
+    """tests/util.bin_reference (the numpy binning the GPU shape sweep compares against) rebuilds the fp32 oracle's own
+    tiles_touched, R, ranges and point_list bit for bit from the oracle's means2D, radii and depths -- incl. a partial
+    last tile row and column, a frame with > 256 tile columns, a single tile, and groups of bit-equal depths."""
+    from util import adversarial_scene, axis_camera, bin_reference
+    if scene == "c3":
+        cloud, _ = synth.make_config("c3", P=20_000)
+        cam = synth.ring_cameras(8, 4.5, 15.0, W, H, 61.0)[5]
+    else:
+        cloud, cls = adversarial_scene()
+        cam = axis_camera(W, H)
+    f = O.forward_from(cloud, cam, render=False)
+    got = bin_reference(f.means2D, f.radii, f.depths, W, H)
+    assert got["R"] == f.num_rendered > 0
+    assert np.array_equal(got["tiles_touched"], f.tiles_touched)
+    assert np.array_equal(got["ranges"], f.ranges)
+    assert np.array_equal(got["point_list"], f.point_list)
+    if scene == "adversarial":   # the tie-break by Gaussian index is exercised
+        d = f.depths[f.point_list]
+        assert np.sum(d[1:] == d[:-1]) >= 50
+    f.close()

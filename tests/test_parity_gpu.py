@@ -24,7 +24,7 @@ import torch
 
 from gaussianeditor_b200 import synth, _lib
 from oracle import cpu_oracle, ref_cuda
-from util import run_ours, rel_l2, cloud_tensors, settings_from
+from util import run_ours, rel_l2, cloud_tensors, settings_from, kernel_options
 
 pytestmark = pytest.mark.gpu
 
@@ -149,8 +149,7 @@ def _small_cases():
 
 @pytest.mark.parametrize("fwd_variant", [0, 1, 2, 3, 4, 5])
 def test_forward_matches_reference_cuda_bit_exact(fwd_variant, reference):
-    _lib.set_option("render_fwd_variant", fwd_variant)
-    try:
+    with kernel_options(render_fwd_variant=fwd_variant):
         for name, cloud, cam, bg in _small_cases():
             ours = run_ours(cloud, cam, bg)
             ref = reference("forward_" + name, lambda: _ref_run(cloud, cam, bg))
@@ -167,14 +166,11 @@ def test_forward_matches_reference_cuda_bit_exact(fwd_variant, reference):
             ref.same("conic_opacity", rec[:, [2, 3, 4, 5]], lambda L: L["state"]["conic_opacity"][vis])
             ref.same("depths", rec[:, 6], lambda L: L["state"]["depths"][vis])
             ref.same("rgb", rec[:, 8:11], lambda L: L["state"]["rgb"][vis])
-    finally:
-        _lib.set_option("render_fwd_variant", 3)
 
 
 @pytest.mark.parametrize("bwd_variant", [0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14])
 def test_backward_matches_reference_cuda(bwd_variant, reference):
-    _lib.set_option("render_bwd_variant", bwd_variant)
-    try:
+    with kernel_options(render_bwd_variant=bwd_variant):
         for name, cloud, cam, bg in _small_cases():
             rng = np.random.default_rng(7)
             dL = rng.uniform(size=(3, cam.image_height, cam.image_width)).astype(np.float32)
@@ -190,8 +186,6 @@ def test_backward_matches_reference_cuda(bwd_variant, reference):
                 err = rel_l2(g, r)
                 assert err <= 1e-4 + 10 * noise, (name, a, err, noise)
                 assert np.abs(g - r).max() <= 1e-3 * r_max + 1e-12, (name, a)
-    finally:
-        _lib.set_option("render_bwd_variant", 4)
 
 
 def test_forward_backward_vs_cpu_oracle():
@@ -540,9 +534,7 @@ def test_binning_variants_match_reference_lists(variant, depth_variant, referenc
     ranges + two own radix passes with the emission fused in (tile_binning.cu, default) -- and both depth orders -- 0: CUB
     radix sort + CUB scan, 1: depth_sort.cu (default) -- must give the reference's point_list / ranges / R bit for bit,
     incl. a partial last tile row/column and a frame with > 256 tile columns."""
-    _lib.set_option("binning_variant", variant)
-    _lib.set_option("depth_sort_variant", depth_variant)
-    try:
+    with kernel_options(binning_variant=variant, depth_sort_variant=depth_variant):
         cloud, _ = synth.make_config("c3", P=80_000)
         for (W, H, k) in [(333, 201, 5), (4160, 48, 1), (1600, 1200, 2)]:
             cam = synth.ring_cameras(8, 4.5, 15.0, W, H, 61.0)[k]
@@ -553,9 +545,6 @@ def test_binning_variants_match_reference_lists(variant, depth_variant, referenc
             ref.same("ranges", v["ranges"], lambda L: L["state"]["ranges"])
             ref.same("point_list", v["point_list"], lambda L: L["state"]["point_list"])
             ref.same("color", ours["color"], lambda L: L["color"])
-    finally:
-        _lib.set_option("binning_variant", 1)
-        _lib.set_option("depth_sort_variant", 1)
 
 
 def test_depth_order_and_offsets_equal_cub_at_full_size():
@@ -564,13 +553,10 @@ def test_depth_order_and_offsets_equal_cub_at_full_size():
     from gaussianeditor_b200.rasterizer import forward_state_views
     cloud, cams = synth.make_config("c3")
     res = {}
-    try:
-        for v in (0, 1):
-            _lib.set_option("depth_sort_variant", v)
+    for v in (0, 1):
+        with kernel_options(depth_sort_variant=v):
             out = run_ours(cloud, cams[2], (0, 0, 0))
-            res[v] = (out["views"]["depth_order"].clone(), out["R"], out["views"]["point_list"].clone())
-    finally:
-        _lib.set_option("depth_sort_variant", 1)
+        res[v] = (out["views"]["depth_order"].clone(), out["R"], out["views"]["point_list"].clone())
     vis = int((out["radii"] > 0).sum())
     assert torch.equal(res[0][0][:vis], res[1][0][:vis])       # among the culled (equal keys) both are index-ordered too:
     assert torch.equal(res[0][0], res[1][0])
