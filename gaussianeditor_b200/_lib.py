@@ -28,6 +28,7 @@ SYMBOLS = [
     "gsr_alpha_image", "gsr_backward_alpha", "gsr_camera_scratch_bytes", "gsr_backward_camera",
     "gsr_sparse_local_bytes", "gsr_sparse_candidate_bytes", "gsr_sparse_view", "gsr_sparse_preprocess", "gsr_sparse_order",
     "gsr_sparse_return", "gsr_sparse_backward_preprocess", "gsr_frame_broadcast", "gsr_peer_barrier",
+    "gsr_backward_depth", "gsr_backward_raw_depth",
 ]
 
 
@@ -146,6 +147,9 @@ def load():
     lib.gsr_backward_camera.restype = C.c_int
     lib.gsr_backward_camera.argtypes = [C.POINTER(Settings), C.POINTER(Cloud), i32, vp, sz, vp, sz, vp, sz, vp, vp, vp, vp,
                                         sz, C.POINTER(Grads), C.POINTER(CameraGrads), vp]
+    lib.gsr_backward_depth.restype = C.c_int
+    lib.gsr_backward_depth.argtypes = [C.POINTER(Settings), C.POINTER(Cloud), i32, vp, sz, vp, sz, vp, sz, vp, vp, vp, vp,
+                                       vp, sz, C.POINTER(Grads), C.POINTER(CameraGrads), vp]
     lib.gsr_alpha_image.restype = C.c_int
     lib.gsr_alpha_image.argtypes = [vp, sz, i32, i32, vp, vp]
     lib.gsr_mark_visible.restype = C.c_int
@@ -189,6 +193,9 @@ def load():
     lib.gsr_backward_raw.restype = C.c_int
     lib.gsr_backward_raw.argtypes = [S, C.POINTER(RawCloud), i32, vp, sz, vp, sz, vp, sz, vp, vp, vp, sz,
                                      C.POINTER(RawGrads), vp]
+    lib.gsr_backward_raw_depth.restype = C.c_int
+    lib.gsr_backward_raw_depth.argtypes = [S, C.POINTER(RawCloud), i32, vp, sz, vp, sz, vp, sz, vp, vp, vp, vp, sz,
+                                           C.POINTER(RawGrads), vp]
     SP = C.POINTER(SparsePlan)
     lib.gsr_sparse_local_bytes.restype = sz; lib.gsr_sparse_local_bytes.argtypes = [i32]
     lib.gsr_sparse_candidate_bytes.restype = sz; lib.gsr_sparse_candidate_bytes.argtypes = [i32, i32]

@@ -198,7 +198,8 @@ int gsr_forward_render_speculative(const gsr_settings* s, const gsr_cloud* c, in
 static int backward_impl(const gsr_settings* s, const gsr_cloud* c, int32_t R, const void* geometry, size_t geometry_bytes,
                          const void* binning, size_t binning_bytes, const void* image, size_t image_bytes,
                          const int32_t* radii, const float* dL_dout_color, const float* dL_dout_alpha, void* scratch,
-                         size_t scratch_bytes, const gsr_grads* gr, void* stream, const gsr_camera_grads* cam = nullptr) {
+                         size_t scratch_bytes, const gsr_grads* gr, void* stream, const gsr_camera_grads* cam = nullptr,
+                         const float* dL_dout_depth = nullptr) {
   int rc = validate_cloud(s, c);
   if (rc) return rc;
   if (!gr || !dL_dout_color) { set_error("grads / dL_dout_color is null"); return GSR_ERR_INVALID; }
@@ -221,7 +222,7 @@ static int backward_impl(const gsr_settings* s, const gsr_cloud* c, int32_t R, c
     cudaError_t e = cudaMemsetAsync(scratch, 0, (size_t)c->P * ACC_STRIDE * sizeof(float), st);
     if (e != cudaSuccess) return check_cuda(e, "scratch memset");
     if (R > 0) {
-      rc = launch_render_bwd(*s, g, b, im, dL_dout_color, (float*)scratch, st, TileOwner(), dL_dout_alpha);
+      rc = launch_render_bwd(*s, g, b, im, dL_dout_color, (float*)scratch, st, TileOwner(), dL_dout_alpha, dL_dout_depth);
       if (rc) return rc;
     }
   }
@@ -233,28 +234,48 @@ static int backward_impl(const gsr_settings* s, const gsr_cloud* c, int32_t R, c
       return GSR_ERR_INVALID;
     }
     CameraBackward cb{cam->dL_dviewmatrix, cam->dL_dprojmatrix, cam->dL_dcampos, (float*)cam->scratch};
-    return launch_preprocess_bwd(*s, *c, g, radii, (const float*)scratch, *gr, st, nullptr, &cb);
+    return launch_preprocess_bwd(*s, *c, g, radii, (const float*)scratch, *gr, st, nullptr, &cb, dL_dout_depth != nullptr);
   }
-  return launch_preprocess_bwd(*s, *c, g, radii, (const float*)scratch, *gr, st);
+  return launch_preprocess_bwd(*s, *c, g, radii, (const float*)scratch, *gr, st, nullptr, nullptr, dL_dout_depth != nullptr);
 }
 
 size_t gsr_camera_scratch_bytes(int32_t P) { return camera_scratch_bytes(P > 0 ? P : 1); }
+
+// P == 0: nothing contributes, the camera gradients are zero (the backward itself returns before any launch)
+static int zero_camera_grads(const gsr_camera_grads* cam, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaSuccess;
+  if (cam->dL_dviewmatrix) e = cudaMemsetAsync(cam->dL_dviewmatrix, 0, 64, st);
+  if (e == cudaSuccess && cam->dL_dprojmatrix) e = cudaMemsetAsync(cam->dL_dprojmatrix, 0, 64, st);
+  if (e == cudaSuccess && cam->dL_dcampos) e = cudaMemsetAsync(cam->dL_dcampos, 0, 12, st);
+  return e == cudaSuccess ? GSR_OK : check_cuda(e, "camera gradient memset");
+}
 
 int gsr_backward_camera(const gsr_settings* s, const gsr_cloud* c, int32_t R, const void* geometry, size_t geometry_bytes,
                         const void* binning, size_t binning_bytes, const void* image, size_t image_bytes,
                         const int32_t* radii, const float* dL_dout_color, const float* dL_dout_alpha, void* scratch,
                         size_t scratch_bytes, const gsr_grads* gr, const gsr_camera_grads* cam, void* stream) {
   if (!cam) { set_error("camera gradients: null struct"); return GSR_ERR_INVALID; }
-  if (c && c->P == 0) {  // nothing contributes: the gradients are zero
-    cudaStream_t st = (cudaStream_t)stream;
-    cudaError_t e = cudaSuccess;
-    if (cam->dL_dviewmatrix) e = cudaMemsetAsync(cam->dL_dviewmatrix, 0, 64, st);
-    if (e == cudaSuccess && cam->dL_dprojmatrix) e = cudaMemsetAsync(cam->dL_dprojmatrix, 0, 64, st);
-    if (e == cudaSuccess && cam->dL_dcampos) e = cudaMemsetAsync(cam->dL_dcampos, 0, 12, st);
-    if (e != cudaSuccess) return check_cuda(e, "camera gradient memset");
+  if (c && c->P == 0) {
+    int rc = zero_camera_grads(cam, stream);
+    if (rc) return rc;
   }
   return backward_impl(s, c, R, geometry, geometry_bytes, binning, binning_bytes, image, image_bytes, radii,
                        dL_dout_color, dL_dout_alpha, scratch, scratch_bytes, gr, stream, cam);
+}
+
+int gsr_backward_depth(const gsr_settings* s, const gsr_cloud* c, int32_t R, const void* geometry, size_t geometry_bytes,
+                       const void* binning, size_t binning_bytes, const void* image, size_t image_bytes,
+                       const int32_t* radii, const float* dL_dout_color, const float* dL_dout_alpha,
+                       const float* dL_dout_depth, void* scratch, size_t scratch_bytes, const gsr_grads* gr,
+                       const gsr_camera_grads* cam, void* stream) {
+  if (!dL_dout_depth) { set_error("depth gradients: dL_dout_depth is null"); return GSR_ERR_INVALID; }
+  if (cam && c && c->P == 0) {
+    int rc = zero_camera_grads(cam, stream);
+    if (rc) return rc;
+  }
+  return backward_impl(s, c, R, geometry, geometry_bytes, binning, binning_bytes, image, image_bytes, radii,
+                       dL_dout_color, dL_dout_alpha, scratch, scratch_bytes, gr, stream, cam, dL_dout_depth);
 }
 
 int gsr_backward(const gsr_settings* s, const gsr_cloud* c, int32_t R, const void* geometry, size_t geometry_bytes,
@@ -336,10 +357,11 @@ int gsr_forward_preprocess_raw(const gsr_settings* s, const gsr_raw_cloud* r, vo
   return first_half(*s, c, g, radii, num_rendered_host, st, true, r->features_rest);
 }
 
-int gsr_backward_raw(const gsr_settings* s, const gsr_raw_cloud* r, int32_t R, const void* geometry,
-                     size_t geometry_bytes, const void* binning, size_t binning_bytes, const void* image,
-                     size_t image_bytes, const int32_t* radii, const float* dL_dout_color, void* scratch,
-                     size_t scratch_bytes, const gsr_raw_grads* gr, void* stream) {
+static int backward_raw_impl(const gsr_settings* s, const gsr_raw_cloud* r, int32_t R, const void* geometry,
+                             size_t geometry_bytes, const void* binning, size_t binning_bytes, const void* image,
+                             size_t image_bytes, const int32_t* radii, const float* dL_dout_color, void* scratch,
+                             size_t scratch_bytes, const gsr_raw_grads* gr, void* stream,
+                             const float* dL_dout_depth = nullptr) {
   gsr_cloud c;
   int rc = raw_to_cloud(s, r, c);
   if (rc) return rc;
@@ -366,7 +388,7 @@ int gsr_backward_raw(const gsr_settings* s, const gsr_raw_cloud* r, int32_t R, c
     cudaError_t e = cudaMemsetAsync(scratch, 0, (size_t)c.P * ACC_STRIDE * sizeof(float), st);
     if (e != cudaSuccess) return check_cuda(e, "scratch memset");
     if (R > 0) {
-      rc = launch_render_bwd(*s, g, b, im, dL_dout_color, (float*)scratch, st);
+      rc = launch_render_bwd(*s, g, b, im, dL_dout_color, (float*)scratch, st, TileOwner(), nullptr, dL_dout_depth);
       if (rc) return rc;
     }
   }
@@ -375,7 +397,25 @@ int gsr_backward_raw(const gsr_settings* s, const gsr_raw_cloud* r, int32_t R, c
   full.dL_dsh = gr->dL_dfeatures_dc; full.dL_dscales = gr->dL_dlog_scales; full.dL_drotations = gr->dL_draw_rotations;
   RawBackward raw{r->features_rest, gr->dL_dfeatures_rest};
   StageScope t(ST_PRE_BWD, st);
-  return launch_preprocess_bwd(*s, c, g, radii, (const float*)scratch, full, st, &raw);
+  return launch_preprocess_bwd(*s, c, g, radii, (const float*)scratch, full, st, &raw, nullptr, dL_dout_depth != nullptr);
+}
+
+int gsr_backward_raw(const gsr_settings* s, const gsr_raw_cloud* r, int32_t R, const void* geometry,
+                     size_t geometry_bytes, const void* binning, size_t binning_bytes, const void* image,
+                     size_t image_bytes, const int32_t* radii, const float* dL_dout_color, void* scratch,
+                     size_t scratch_bytes, const gsr_raw_grads* gr, void* stream) {
+  return backward_raw_impl(s, r, R, geometry, geometry_bytes, binning, binning_bytes, image, image_bytes, radii,
+                           dL_dout_color, scratch, scratch_bytes, gr, stream);
+}
+
+int gsr_backward_raw_depth(const gsr_settings* s, const gsr_raw_cloud* r, int32_t R, const void* geometry,
+                           size_t geometry_bytes, const void* binning, size_t binning_bytes, const void* image,
+                           size_t image_bytes, const int32_t* radii, const float* dL_dout_color,
+                           const float* dL_dout_depth, void* scratch, size_t scratch_bytes, const gsr_raw_grads* gr,
+                           void* stream) {
+  if (!dL_dout_depth) { set_error("depth gradients: dL_dout_depth is null"); return GSR_ERR_INVALID; }
+  return backward_raw_impl(s, r, R, geometry, geometry_bytes, binning, binning_bytes, image, image_bytes, radii,
+                           dL_dout_color, scratch, scratch_bytes, gr, stream, dL_dout_depth);
 }
 
 // ---- Gaussian-sharded multi-GPU path ---------------------------------------------------------------------

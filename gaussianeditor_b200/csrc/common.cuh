@@ -90,6 +90,7 @@ void carve_image(void* base, int W, int H, ImageWS& ws);
 
 // Backward scratch: per-Gaussian accumulators of the nine 2-D gradients (+3 pad -> 48 B, 16-B aligned):
 //   [0..2] dL/dcolor  [3..4] dL/dmean2D  [5..7] dL/dconic (a,b,c)  [8] dL/dopacity
+//   [9] dL/d(view depth), written only by the depth-gradient backward (gsr_backward_depth), zero otherwise
 constexpr int ACC_STRIDE = 12;
 
 // ---- options -----------------------------------------------------------------------------------------
@@ -150,13 +151,14 @@ int launch_render_fwd(const gsr_settings& s, const GeometryWS& g, const BinningW
                       float* out_color, float* out_depth, cudaStream_t st, const TileOwner& own = TileOwner());
 int launch_render_bwd(const gsr_settings& s, const GeometryWS& g, const BinningWS& b, const ImageWS& im,
                       const float* dL_dpix, float* acc, cudaStream_t st, const TileOwner& own = TileOwner(),
-                      const float* dL_dalpha_img = nullptr);
+                      const float* dL_dalpha_img = nullptr, const float* dL_ddepth = nullptr);
 // raw != nullptr: RAW variant -- gradients w.r.t. the raw parameters (gr.dL_dsh = d features_dc, raw->dL_dfeatures_rest)
 struct RawBackward {
   const float* features_rest;
   float* dL_dfeatures_rest;
 };
 // cam != nullptr: also dL/dviewmatrix [16], dL/dprojmatrix [16], dL/dcampos [3] (opt-in; scratch = camera_scratch_bytes(P))
+// depth: acc slot 9 holds dL/d(view depth) (gsr_backward_depth) and enters dL/dt.z
 struct CameraBackward {
   float* dL_dviewmatrix;
   float* dL_dprojmatrix;
@@ -166,7 +168,7 @@ struct CameraBackward {
 size_t camera_scratch_bytes(int P);
 int launch_preprocess_bwd(const gsr_settings& s, const gsr_cloud& c, const GeometryWS& g, const int32_t* radii,
                           const float* acc, const gsr_grads& gr, cudaStream_t st, const RawBackward* raw = nullptr,
-                          const CameraBackward* cam = nullptr);
+                          const CameraBackward* cam = nullptr, bool depth = false);
 // out_alpha[i] = 1 - final_T[i]  (the reference keeps final_T as ImageState::accum_alpha, rasterizer_impl.h:50)
 int launch_alpha_image(const float* final_T, size_t n, float* out_alpha, cudaStream_t st);
 int launch_mark_visible(int P, const float* means3D, const float* viewmatrix, uint8_t* present, cudaStream_t st);

@@ -72,6 +72,7 @@ struct PbArgs {
   const float* features_rest;
   float* dL_dfeatures_rest;
   float* cam_partial;  // CAM variant: [nblocks, CAM_STRIDE] block partial sums of the camera gradients
+  int depth;           // acc slot 9 holds dL/d(view depth) (gsr_backward_depth): add it to dL/dt.z
 };
 
 __device__ __forceinline__ M3 quat_to_R(float r, float x, float y, float z) {
@@ -153,7 +154,7 @@ __global__ void __launch_bounds__(PB_THREADS) preprocess_bwd_kernel(const PbArgs
     const float4* ap = reinterpret_cast<const float4*>(a.acc + (size_t)idx * ACC_STRIDE);
     acc0 = __ldg(ap);      // dcolor.rgb, dmean2D.x
     acc1 = __ldg(ap + 1);  // dmean2D.y, dconic.a, dconic.b, dconic.c
-    acc2 = __ldg(ap + 2);  // dopacity
+    acc2 = __ldg(ap + 2);  // dopacity, dL/d(view depth) (slot 9; zero unless the depth gradient was requested)
     mean = make_float3(a.means3D[3 * idx], a.means3D[3 * idx + 1], a.means3D[3 * idx + 2]);
 
     // ---- 3-D covariance (recomputed; forward.cu:118-152) ----
@@ -249,8 +250,11 @@ __global__ void __launch_bounds__(PB_THREADS) preprocess_bwd_kernel(const PbArgs
       const float tz = 1.f / t.z, tz2 = tz * tz, tz3 = tz2 * tz;
       const float dL_dtx = x_grad_mul * -a.h_x * tz2 * dL_dJ02;
       const float dL_dty = y_grad_mul * -a.h_y * tz2 * dL_dJ12;
-      const float dL_dtz = -a.h_x * tz2 * dL_dJ00 - a.h_y * tz2 * dL_dJ11 + (2 * a.h_x * t.x) * tz3 * dL_dJ02 +
-                           (2 * a.h_y * t.y) * tz3 * dL_dJ12;
+      float dL_dtz = -a.h_x * tz2 * dL_dJ00 - a.h_y * tz2 * dL_dJ11 + (2 * a.h_x * t.x) * tz3 * dL_dJ02 +
+                     (2 * a.h_y * t.y) * tz3 * dL_dJ12;
+      // the depth image reads d_i = t.z (unclamped): its gradient joins dL/dt.z and from there the mean, cov3D_precomp,
+      // RAW and camera paths below. A uniform branch, not `+ 0`: without the flag the gradients stay bit-identical.
+      if (a.depth) dL_dtz += acc2.y;
       // transformVec4x3Transpose (auxiliary.h:89-97)
       dmean[0] = vm[0] * dL_dtx + vm[1] * dL_dty + vm[2] * dL_dtz;
       dmean[1] = vm[4] * dL_dtx + vm[5] * dL_dty + vm[6] * dL_dtz;
@@ -545,8 +549,9 @@ size_t camera_scratch_bytes(int P) { return align_up((size_t)((P + PB_THREADS - 
 
 int launch_preprocess_bwd(const gsr_settings& s, const gsr_cloud& c, const GeometryWS& g, const int32_t* radii,
                           const float* acc, const gsr_grads& gr, cudaStream_t st, const RawBackward* raw,
-                          const CameraBackward* cam) {
+                          const CameraBackward* cam, bool depth) {
   PbArgs a;
+  a.depth = depth ? 1 : 0;
   a.cam_partial = cam ? cam->scratch : nullptr;
   a.opacities = c.opacities;
   a.features_rest = raw ? raw->features_rest : nullptr;

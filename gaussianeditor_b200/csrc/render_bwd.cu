@@ -43,6 +43,8 @@ struct BwdArgs {
   float* acc;  // [P, ACC_STRIDE]
   int own_stride, own_phase;  // tile-row ownership (1, 0 = all tiles)
 };
+// The DEPTH kernels take dL/d(depth image) [H*W] (gsr_backward_depth) as a separate last kernel parameter: BwdArgs keeps
+// its layout, so the instantiations without depth compile to exactly the code they had before the depth gradient.
 
 // One (pixel, splat) hit. `ar` tracks the reference's accum_rec (backward.cu:515) dotted with dL_dpixel, updated
 // eagerly; `bgT` = T_final * (bg . dL_dpixel).
@@ -52,9 +54,15 @@ struct BwdArgs {
 // and turned into the reference's quantities once per (tile, splat) by finish_sums() -- the per-splat factors
 // (conic, opacity, 0.5*W, 0.5*H) are constant over the pixels, so this is the same sum with the common factor
 // pulled out (8 instead of 17 operations per hit).
+//
+// DEPTH (gsr_backward_depth): the depth image D = sum d_i*alpha_i*T_i is a fourth colour channel without a background
+// term, with the record's view depth d_i as its colour and dD = dL/dD(pixel) as its upstream gradient. It joins the
+// scalar recurrence (s += d_i*dD) and adds one more per-Gaussian sum, g[9] = sum alpha*T*dD = dL/dd_i (acc slot 9).
 struct PixState {
   float T, ar, d0, d1, d2, bgT;   // ar = accum_rec . dL_dpixel (scalar; see hit_update)
+  float dD;                       // DEPTH only: dL/d(depth image) at this pixel
 };
+constexpr int nsums(bool depth) { return depth ? 10 : 9; }
 
 // What multiplies dT_final/dalpha_i = -T_final/(1-alpha_i) in dL/dalpha_i: the background term of the colour
 // (backward.cu:505-511: bg . dL_dpixel) and, when the caller asked for the alpha image A = 1 - T_final, -dL/dA.
@@ -64,8 +72,9 @@ __device__ __forceinline__ float bg_term(const BwdArgs& a, size_t pix_id, float 
   return t;
 }
 
+template <bool DEPTH>
 __device__ __forceinline__ void hit_update(PixState& p, float* g, float dx, float dy, float G, float alpha, float o,
-                                           float c0, float c1, float c2) {
+                                           float c0, float c1, float c2, float depth) {
   const float oma = 1.f - alpha;
   float rcp;  // 1-alpha is in [0.01, 1]: the bare MUFU.RCP (<= 1 ulp here) needs no range fix-up
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rcp) : "f"(oma));
@@ -76,11 +85,13 @@ __device__ __forceinline__ void hit_update(PixState& p, float* g, float dx, floa
   // sum_ch (c_ch - accum_rec_ch) * dL_dpixel_ch. Only that dot product is ever used, and the recurrence
   // accum_rec' = alpha*c + (1-alpha)*accum_rec is linear, so the scalar ar = accum_rec . dL_dpixel obeys
   // ar' = ar + alpha*(c.dL_dpixel - ar): one state variable and 5 operations instead of three and 9.
-  const float s = fmaf(c2, p.d2, fmaf(c1, p.d1, c0 * p.d0));
+  float s = fmaf(c2, p.d2, fmaf(c1, p.d1, c0 * p.d0));
+  if constexpr (DEPTH) s = fmaf(depth, p.dD, s);  // the depth channel: colour d_i, no background
   float dL_dalpha = s - p.ar;
   g[0] = fmaf(dchannel_dcolor, p.d0, g[0]);
   g[1] = fmaf(dchannel_dcolor, p.d1, g[1]);
   g[2] = fmaf(dchannel_dcolor, p.d2, g[2]);
+  if constexpr (DEPTH) g[9] = fmaf(dchannel_dcolor, p.dD, g[9]);
   p.ar = fmaf(alpha, dL_dalpha, p.ar);
   dL_dalpha = fmaf(dL_dalpha, p.T, -p.bgT * rcp);
   const float w = (o * dL_dalpha) * G;  // dL_dG * G
@@ -100,6 +111,7 @@ __device__ __forceinline__ void hit_update(PixState& p, float* g, float dx, floa
 //   j<3: tot | j=3: -(A*s_x + B*s_y)*0.5W | j=4: -(C*s_y + B*s_x)*0.5H | j=5..7: -0.5*tot | opacity: sw / o
 struct LaneRole {
   bool is_x, is_y, writer, opac;  // moment-3 group, moment-4 group, lane that issues the atomic, opacity lane
+  bool dep;                       // DEPTH: the lane that adds dL/d(view depth) into slot 9 (neither a writer nor lane 1)
   float kconst;                   // 1 for the colour groups, -0.5 for the conic groups
   int slot;
 };
@@ -110,11 +122,13 @@ __device__ __forceinline__ LaneRole lane_role(int lane) {
   r.is_y = r.slot == 4;
   r.writer = (lane & 3) == 0;
   r.opac = lane == 1;
+  r.dep = lane == 2;
   r.kconst = r.slot < 3 ? 1.0f : -0.5f;
   return r;
 }
-__device__ __forceinline__ void finish_and_add(float* dst, float tot, float sw, const LaneRole& role, float A, float B,
-                                               float C, float o, float ddelx_dx, float ddely_dy) {
+template <bool DEPTH>
+__device__ __forceinline__ void finish_and_add(float* dst, float tot, float sw, float sd, const LaneRole& role, float A,
+                                               float B, float C, float o, float ddelx_dx, float ddely_dy) {
   const float other = __shfl_xor_sync(0xffffffffu, tot, 28);  // s_x <-> s_y between lanes 12..15 and 16..19
   const float nBx = -B * ddelx_dx, nBy = -B * ddely_dy;
   const float ka = role.is_x ? -A * ddelx_dx : (role.is_y ? -C * ddely_dy : role.kconst);
@@ -122,12 +136,16 @@ __device__ __forceinline__ void finish_and_add(float* dst, float tot, float sw, 
   const float v = fmaf(kb, other, ka * tot);
   if (role.writer) atomicAdd(dst + role.slot, v);
   if (role.opac) atomicAdd(dst + 8, __fdividef(sw, o));  // dL/dopacity = sum G*dL_dalpha = (sum w) / o
+  if constexpr (DEPTH) {
+    if (role.dep) atomicAdd(dst + 9, sd);  // dL/d(view depth) = sum alpha*T*dL/dD
+  }
 }
 
 // Sum nine per-lane values over the warp. g[0..7] go through a transposing butterfly: after it, lane 4*j (and
 // its three neighbours) holds the warp total of g[j]; g[8] takes a plain butterfly. Returns this lane's total of
-// value (lane>>2), and the total of g[8] in `g8`.
-__device__ __forceinline__ float warp_sum9(const float* g, int lane, float& g8) {
+// value (lane>>2), and the total of g[8] in `g8`. DEPTH: g[9] takes a plain butterfly too, its total in `g9`.
+template <bool DEPTH>
+__device__ __forceinline__ float warp_sum9(const float* g, int lane, float& g8, float& g9) {
   const unsigned F = 0xffffffffu;
   float a[4], b[2], c;
   {
@@ -160,6 +178,12 @@ __device__ __forceinline__ float warp_sum9(const float* g, int lane, float& g8) 
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(F, t, o);
   g8 = t;
+  if constexpr (DEPTH) {
+    float d = g[9];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) d += __shfl_xor_sync(F, d, o);
+    g9 = d;
+  }
   return c;
 }
 
@@ -168,8 +192,9 @@ __device__ __forceinline__ float warp_sum9(const float* g, int lane, float& g8) 
 // ------------------------------------------------------------------------------------------------------
 constexpr int BW_WARPS = 4;
 
-template <int NSB>
-__global__ void __launch_bounds__(BW_WARPS * 32) render_bwd_warp_kernel(const BwdArgs a, const int ntiles) {
+template <int NSB, bool DEPTH = false>
+__global__ void __launch_bounds__(BW_WARPS * 32) render_bwd_warp_kernel(const BwdArgs a, const int ntiles,
+                                                                        const float* dL_ddepth) {
   __shared__ float4 s_stage[BW_WARPS][3][32];
   __shared__ uint32_t s_id[BW_WARPS][32];
   constexpr int PARTS = 8 / NSB;
@@ -200,7 +225,7 @@ __global__ void __launch_bounds__(BW_WARPS * 32) render_bwd_warp_kernel(const Bw
     const int kg = part * NSB + k;
     const int px = tx * TILE + 8 * (kg & 1) + lx, py = ty * TILE + 4 * (kg >> 1) + ly;
     PixState p;
-    p.T = 0.f; p.ar = 0.f; p.d0 = p.d1 = p.d2 = 0.f; p.bgT = 0.f;
+    p.T = 0.f; p.ar = 0.f; p.d0 = p.d1 = p.d2 = 0.f; p.bgT = 0.f; p.dD = 0.f;
     nc[k] = 0;
     if (px < a.W && py < a.H) {
       const size_t pix_id = (size_t)a.W * py + px;
@@ -210,6 +235,7 @@ __global__ void __launch_bounds__(BW_WARPS * 32) render_bwd_warp_kernel(const Bw
       p.d1 = a.dL_dpix[HW + pix_id];
       p.d2 = a.dL_dpix[2 * HW + pix_id];
       p.bgT = Tf * bg_term(a, pix_id, bg0, bg1, bg2, p);
+      if constexpr (DEPTH) p.dD = dL_ddepth[pix_id];
       nc[k] = a.n_contrib[pix_id];
     }
     ps[k] = p;
@@ -267,9 +293,9 @@ __global__ void __launch_bounds__(BW_WARPS * 32) render_bwd_warp_kernel(const Bw
         dyv[r] = s0.y - (fy + 4.0f * (float)(part * (NSB / 2) + r));
         t0[r] = __fmul_rn(__fmul_rn(dyv[r], s1.x), dyv[r]);
       }
-      float g[9];
+      float g[nsums(DEPTH)];
 #pragma unroll
-      for (int i = 0; i < 9; i++) g[i] = 0.f;
+      for (int i = 0; i < nsums(DEPTH); i++) g[i] = 0.f;
       bool any = false;
 #pragma unroll
       for (int k = 0; k < NSB; k++) {
@@ -283,12 +309,13 @@ __global__ void __launch_bounds__(BW_WARPS * 32) render_bwd_warp_kernel(const Bw
         const float alpha = fminf(0.99f, __fmul_rn(s1.y, G));
         if (alpha < 1.0f / 255.0f) continue;
         any = true;
-        hit_update(ps[k], g, dx, dy, G, alpha, s1.y, s2.x, s2.y, s2.z);
+        hit_update<DEPTH>(ps[k], g, dx, dy, G, alpha, s1.y, s2.x, s2.y, s2.z, s1.z);
       }
       if (__any_sync(0xffffffffu, any)) {
-        float m8;
-        const float tot = warp_sum9(g, lane, m8);
-        finish_and_add(a.acc + (size_t)sid[j] * ACC_STRIDE, tot, m8, role, s0.z, s0.w, s1.x, s1.y, ddelx_dx, ddely_dy);
+        float m8, m9;
+        const float tot = warp_sum9<DEPTH>(g, lane, m8, m9);
+        finish_and_add<DEPTH>(a.acc + (size_t)sid[j] * ACC_STRIDE, tot, m8, m9, role, s0.z, s0.w, s1.x, s1.y, ddelx_dx,
+                              ddely_dy);
       }
     }
     __syncwarp();
@@ -309,8 +336,9 @@ __device__ __forceinline__ float ex2_approx(float x) {
   return y;
 }
 
-template <int NSB, int MINB, bool SKIP = false, bool MASKSKIP = false>
-__global__ void __launch_bounds__(BW_WARPS * 32, MINB) render_bwd_flat_kernel(const BwdArgs a, const int ntiles) {
+template <int NSB, int MINB, bool SKIP = false, bool MASKSKIP = false, bool DEPTH = false>
+__global__ void __launch_bounds__(BW_WARPS * 32, MINB) render_bwd_flat_kernel(const BwdArgs a, const int ntiles,
+                                                                                 const float* dL_ddepth) {
   __shared__ float4 s_stage[BW_WARPS][3][32];
   __shared__ uint32_t s_id[BW_WARPS][32];
   constexpr int PARTS = 8 / NSB;
@@ -341,7 +369,7 @@ __global__ void __launch_bounds__(BW_WARPS * 32, MINB) render_bwd_flat_kernel(co
     const int kg = part * NSB + k;
     const int px = tx * TILE + 8 * (kg & 1) + lx, py = ty * TILE + 4 * (kg >> 1) + ly;
     PixState p;
-    p.T = 0.f; p.ar = 0.f; p.d0 = p.d1 = p.d2 = 0.f; p.bgT = 0.f;
+    p.T = 0.f; p.ar = 0.f; p.d0 = p.d1 = p.d2 = 0.f; p.bgT = 0.f; p.dD = 0.f;
     nc[k] = 0;
     if (px < a.W && py < a.H) {
       const size_t pix_id = (size_t)a.W * py + px;
@@ -351,6 +379,7 @@ __global__ void __launch_bounds__(BW_WARPS * 32, MINB) render_bwd_flat_kernel(co
       p.d1 = a.dL_dpix[HW + pix_id];
       p.d2 = a.dL_dpix[2 * HW + pix_id];
       p.bgT = Tf * bg_term(a, pix_id, bg0, bg1, bg2, p);
+      if constexpr (DEPTH) p.dD = dL_ddepth[pix_id];
       nc[k] = a.n_contrib[pix_id];
     }
     ps[k] = p;
@@ -442,19 +471,20 @@ __global__ void __launch_bounds__(BW_WARPS * 32, MINB) render_bwd_flat_kernel(co
         if (SKIP && __any_sync(0xffffffffu, ok)) hitk |= 1u << k;
       }
       if (SKIP ? hitk == 0 : !__any_sync(0xffffffffu, anyhit)) continue;
-      float g[9];
+      float g[nsums(DEPTH)];
 #pragma unroll
-      for (int i = 0; i < 9; i++) g[i] = 0.f;
+      for (int i = 0; i < nsums(DEPTH); i++) g[i] = 0.f;
 #pragma unroll
       for (int k = 0; k < NSB; k++) {
         // (alpha, G) = (0, 0) makes every update below an exact no-op: 1/(1-0) = 1, +0 contributions
         if (SKIP && !((hitk >> k) & 1u)) continue;
         if (MASKSKIP && !((m >> k) & 1u)) continue;
-        hit_update(ps[k], g, dxv[k & 1], dyv[k >> 1], G[k], al[k], s1.y, s2.x, s2.y, s2.z);
+        hit_update<DEPTH>(ps[k], g, dxv[k & 1], dyv[k >> 1], G[k], al[k], s1.y, s2.x, s2.y, s2.z, s1.z);
       }
-      float m8;
-      const float tot = warp_sum9(g, lane, m8);
-      finish_and_add(a.acc + (size_t)sid[j] * ACC_STRIDE, tot, m8, role, s0.z, s0.w, s1.x, s1.y, ddelx_dx, ddely_dy);
+      float m8, m9;
+      const float tot = warp_sum9<DEPTH>(g, lane, m8, m9);
+      finish_and_add<DEPTH>(a.acc + (size_t)sid[j] * ACC_STRIDE, tot, m8, m9, role, s0.z, s0.w, s1.x, s1.y, ddelx_dx,
+                            ddely_dy);
     }
     __syncwarp();
   }
@@ -463,7 +493,8 @@ __global__ void __launch_bounds__(BW_WARPS * 32, MINB) render_bwd_flat_kernel(co
 // ------------------------------------------------------------------------------------------------------
 // Variant 0: CTA per tile, one pixel per thread, butterfly reduction of the nine sums per splat
 // ------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(TILE_PIX) render_bwd_cta_kernel(const BwdArgs a) {
+template <bool DEPTH = false>
+__global__ void __launch_bounds__(TILE_PIX) render_bwd_cta_kernel(const BwdArgs a, const float* dL_ddepth) {
   __shared__ float4 s_q0[TILE_PIX], s_q1[TILE_PIX], s_q2[TILE_PIX];
   __shared__ uint32_t s_ids[TILE_PIX];
   const int tile = blockIdx.y * a.gx + blockIdx.x;
@@ -478,13 +509,14 @@ __global__ void __launch_bounds__(TILE_PIX) render_bwd_cta_kernel(const BwdArgs 
   const size_t HW = (size_t)a.H * a.W;
 
   PixState p;
-  p.T = 0.f; p.ar = 0.f; p.d0 = p.d1 = p.d2 = 0.f; p.bgT = 0.f;
+  p.T = 0.f; p.ar = 0.f; p.d0 = p.d1 = p.d2 = 0.f; p.bgT = 0.f; p.dD = 0.f;
   uint32_t nc = 0;
   if (inside) {
     const float Tf = a.final_T[pix_id];
     p.T = Tf;
     p.d0 = a.dL_dpix[pix_id]; p.d1 = a.dL_dpix[HW + pix_id]; p.d2 = a.dL_dpix[2 * HW + pix_id];
     p.bgT = Tf * bg_term(a, pix_id, a.bg[0], a.bg[1], a.bg[2], p);
+    if constexpr (DEPTH) p.dD = dL_ddepth[pix_id];
     nc = a.n_contrib[pix_id];
   }
   const float ddelx_dx = 0.5f * a.W, ddely_dy = 0.5f * a.H;
@@ -506,9 +538,9 @@ __global__ void __launch_bounds__(TILE_PIX) render_bwd_cta_kernel(const BwdArgs 
       const float4 q0 = s_q0[j], q1 = s_q1[j];
       const float dx = q0.x - pixf.x, dy = q0.y - pixf.y;
       const float power = splat_power(dx, dy, q0.z, q0.w, q1.x);
-      float g[9];
+      float g[nsums(DEPTH)];
 #pragma unroll
-      for (int i = 0; i < 9; i++) g[i] = 0.f;
+      for (int i = 0; i < nsums(DEPTH); i++) g[i] = 0.f;
       bool hit = false;
       if (!(power > 0.0f) && spos <= nc) {
         const float G = expf(power);
@@ -516,15 +548,56 @@ __global__ void __launch_bounds__(TILE_PIX) render_bwd_cta_kernel(const BwdArgs 
         if (!(alpha < 1.0f / 255.0f)) {
           hit = true;
           const float4 q2 = s_q2[j];
-          hit_update(p, g, dx, dy, G, alpha, q1.y, q2.x, q2.y, q2.z);
+          hit_update<DEPTH>(p, g, dx, dy, G, alpha, q1.y, q2.x, q2.y, q2.z, q1.z);
         }
       }
       if (__any_sync(0xffffffffu, hit)) {
-        float m8;
-        const float tot = warp_sum9(g, lane, m8);
-        finish_and_add(a.acc + (size_t)s_ids[j] * ACC_STRIDE, tot, m8, role, q0.z, q0.w, q1.x, q1.y, ddelx_dx, ddely_dy);
+        float m8, m9;
+        const float tot = warp_sum9<DEPTH>(g, lane, m8, m9);
+        finish_and_add<DEPTH>(a.acc + (size_t)s_ids[j] * ACC_STRIDE, tot, m8, m9, role, q0.z, q0.w, q1.x, q1.y, ddelx_dx,
+                              ddely_dy);
       }
     }
+  }
+}
+
+// One launch of render_bwd_variant v (see Options::render_bwd_variant); DEPTH picks the instantiation that also
+// back-propagates the depth image. Every variant exists in both forms, so the variant option never drops dL/dD.
+template <bool DEPTH>
+void launch_variant(int v, const BwdArgs& a, int ntiles, const float* dL_ddepth, cudaStream_t st) {
+  if (v == 0) {
+    render_bwd_cta_kernel<DEPTH><<<dim3(a.gx, a.gy), dim3(TILE, TILE), 0, st>>>(a, dL_ddepth);
+  } else if (v == 2) {
+    const int warps = ntiles * 2;
+    render_bwd_warp_kernel<4, DEPTH><<<(warps + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 3) {
+    const int warps = ntiles * 4;
+    render_bwd_warp_kernel<2, DEPTH><<<(warps + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 4) {
+    render_bwd_flat_kernel<4, 1, false, false, DEPTH><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 5) {
+    render_bwd_flat_kernel<4, 6, false, false, DEPTH><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 6) {
+    render_bwd_flat_kernel<2, 1, false, false, DEPTH><<<(ntiles * 4 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 7) {
+    render_bwd_flat_kernel<8, 1, false, false, DEPTH><<<(ntiles + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 8) {
+    render_bwd_flat_kernel<4, 1, true, false, DEPTH><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 9) {
+    render_bwd_flat_kernel<8, 1, true, false, DEPTH><<<(ntiles + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 12) {  // register caps: 5 / 6 CTAs per SM, with and without the hit-skip
+    render_bwd_flat_kernel<4, 5, false, false, DEPTH><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 13) {
+    render_bwd_flat_kernel<4, 6, true, false, DEPTH><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 14) {
+    // the DEPTH instantiation fits the same cap without spilling (96 registers, 5 CTAs/SM)
+    render_bwd_flat_kernel<4, 5, true, false, DEPTH><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 10) {  // variant 4 + sub-blocks outside the splat's mask skipped with warp-uniform branches
+    render_bwd_flat_kernel<4, 1, false, true, DEPTH><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else if (v == 11) {  // the same for the quarter-tile mapping
+    render_bwd_flat_kernel<2, 1, false, true, DEPTH><<<(ntiles * 4 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
+  } else {
+    render_bwd_warp_kernel<8, DEPTH><<<(ntiles + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles, dL_ddepth);
   }
 }
 
@@ -532,7 +605,7 @@ __global__ void __launch_bounds__(TILE_PIX) render_bwd_cta_kernel(const BwdArgs 
 
 int launch_render_bwd(const gsr_settings& s, const GeometryWS& g, const BinningWS& b, const ImageWS& im,
                       const float* dL_dpix, float* acc, cudaStream_t st, const TileOwner& own,
-                      const float* dL_dalpha_img) {
+                      const float* dL_dalpha_img, const float* dL_ddepth) {
   BwdArgs a;
   a.dL_dalpha_img = dL_dalpha_img;
   a.own_stride = own.stride; a.own_phase = own.phase;
@@ -544,39 +617,10 @@ int launch_render_bwd(const gsr_settings& s, const GeometryWS& g, const BinningW
   if (ntiles == 0) return GSR_OK;
   int v = g_opt.render_bwd_variant;
   if (v == 0 && own.stride != 1) v = 4;  // the CTA-per-tile kernel maps blockIdx to tiles directly: single-GPU only
-  if (v == 0) {
-    render_bwd_cta_kernel<<<dim3(a.gx, a.gy), dim3(TILE, TILE), 0, st>>>(a);
-  } else if (v == 2) {
-    const int warps = ntiles * 2;
-    render_bwd_warp_kernel<4><<<(warps + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 3) {
-    const int warps = ntiles * 4;
-    render_bwd_warp_kernel<2><<<(warps + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 4) {
-    render_bwd_flat_kernel<4, 1><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 5) {
-    render_bwd_flat_kernel<4, 6><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 6) {
-    render_bwd_flat_kernel<2, 1><<<(ntiles * 4 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 7) {
-    render_bwd_flat_kernel<8, 1><<<(ntiles + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 8) {
-    render_bwd_flat_kernel<4, 1, true><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 9) {
-    render_bwd_flat_kernel<8, 1, true><<<(ntiles + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 12) {  // register caps: 5 / 6 CTAs per SM, with and without the hit-skip
-    render_bwd_flat_kernel<4, 5><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 13) {
-    render_bwd_flat_kernel<4, 6, true><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 14) {
-    render_bwd_flat_kernel<4, 5, true><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 10) {  // variant 4 + sub-blocks outside the splat's mask skipped with warp-uniform branches
-    render_bwd_flat_kernel<4, 1, false, true><<<(ntiles * 2 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else if (v == 11) {  // the same for the quarter-tile mapping
-    render_bwd_flat_kernel<2, 1, false, true><<<(ntiles * 4 + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  } else {
-    render_bwd_warp_kernel<8><<<(ntiles + BW_WARPS - 1) / BW_WARPS, BW_WARPS * 32, 0, st>>>(a, ntiles);
-  }
+  if (dL_ddepth != nullptr)
+    launch_variant<true>(v, a, ntiles, dL_ddepth, st);
+  else
+    launch_variant<false>(v, a, ntiles, nullptr, st);
   g_launches++;
   return check_launch("render_bwd", s.debug != 0, st);
 }

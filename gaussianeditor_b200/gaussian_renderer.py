@@ -63,7 +63,7 @@ def _python_sh_colors(pc, camera_center) -> torch.Tensor:
 
 
 def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, scaling_modifier=1.0, override_color=None,
-           fused_activations: bool = False):
+           fused_activations: bool = False, depth_grad: bool = False):
     """Render the scene; background tensor must be on the GPU. Returns the reference's dictionary:
     render [3,H,W], viewspace_points [P,3] (grad sink for densification), visibility_filter, radii, depth_3dgs.
 
@@ -71,7 +71,11 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, scaling_modifier=
     (``pc._opacity, pc._features_dc, pc._features_rest, pc._scaling, pc._rotation``) to the rasterizer, which applies
     sigmoid / exp / normalize and reads the SH row from the two feature arrays inside its preprocess kernels: the
     per-render PyTorch prologue (five elementwise kernels, a [P,16,3] ``torch.cat``) and its autograd epilogue go away.
-    Only valid for the plain SH path (no override colour, no Python-side SH / covariance)."""
+    Only valid for the plain SH path (no override colour, no Python-side SH / covariance).
+
+    ``depth_grad=True`` (opt-in, not in the reference) makes ``depth_3dgs`` differentiable on both paths (a depth loss
+    then also reaches ``viewspace_points.grad``, which densification reads); without it, as in the reference, a loss on
+    the depth trains nothing."""
     xyz = pc.get_xyz
     # gradient sink for the 2-D means: densification reads its .grad (gaussian_renderer/__init__.py:60-69)
     screenspace_points = torch.zeros_like(xyz, requires_grad=True) + 0
@@ -80,7 +84,8 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, scaling_modifier=
     except Exception:
         pass
     rasterizer = GaussianRasterizer(
-        raster_settings=_settings_for(viewpoint_camera, bg_color, scaling_modifier, pc.active_sh_degree))
+        raster_settings=_settings_for(viewpoint_camera, bg_color, scaling_modifier, pc.active_sh_degree),
+        depth_grad=depth_grad)
     python_sh = getattr(pipe, "convert_SHs_python", False)
     python_cov = getattr(pipe, "compute_cov3D_python", False)
 

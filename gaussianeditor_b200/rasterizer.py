@@ -209,13 +209,14 @@ def _forward_impl(means3D, sh, colors_precomp, opacities, scales, rotations, cov
 
 
 def rasterize_gaussians(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                        raster_settings, return_alpha=False, camera_grad=False):
+                        raster_settings, return_alpha=False, camera_grad=False, depth_grad=False):
     if camera_grad:   # the camera arrays become autograd inputs of the node (they are read from the settings as usual)
         rs = raster_settings
         return _RasterizeGaussians.apply(means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
-                                         cov3Ds_precomp, rs, return_alpha, rs.viewmatrix, rs.projmatrix, rs.campos)
+                                         cov3Ds_precomp, rs, return_alpha, depth_grad, rs.viewmatrix, rs.projmatrix,
+                                         rs.campos)
     return _RasterizeGaussians.apply(means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
-                                     cov3Ds_precomp, raster_settings, return_alpha)
+                                     cov3Ds_precomp, raster_settings, return_alpha, depth_grad)
 
 
 def _alpha_image(lib, state, device):
@@ -231,12 +232,13 @@ def _alpha_image(lib, state, device):
 class _RasterizeGaussians(torch.autograd.Function):
     @staticmethod
     def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                raster_settings, return_alpha=False, viewmatrix=None, projmatrix=None, campos=None):
+                raster_settings, return_alpha=False, depth_grad=False, viewmatrix=None, projmatrix=None, campos=None):
         color, depth, state, inputs = _forward_impl(means3D, sh, colors_precomp, opacities, scales, rotations,
                                                     cov3Ds_precomp, raster_settings)
         ctx.raster_settings = raster_settings
         ctx.camera_grad = viewmatrix is not None
-        ctx.n_inputs = 10 + (3 if ctx.camera_grad else 0)
+        ctx.depth_grad = bool(depth_grad)
+        ctx.n_inputs = 11 + (3 if ctx.camera_grad else 0)
         ctx.state = state
         ctx.save_for_backward(*inputs, state.radii, state.geom, state.binning, state.img)
         ctx.mark_non_differentiable(state.radii)
@@ -271,18 +273,28 @@ class _RasterizeGaussians(torch.autograd.Function):
                 gr = _lib.Grads(_ptr(dL_dmeans3D), _ptr(dL_dmeans2D), _ptr(dL_dcolors), _ptr(dL_dopacity),
                                 _ptr(dL_dcov3D), _ptr(dL_dsh), _ptr(dL_dscales), _ptr(dL_drotations))
                 st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+                cam = None
                 if ctx.camera_grad:
                     d_view = torch.empty(16, **f32); d_proj = torch.empty(16, **f32); d_cam = torch.empty(3, **f32)
                     cbytes = lib.gsr_camera_scratch_bytes(P)
                     cscratch = torch.empty(cbytes, dtype=torch.uint8, device=device)
                     cam = _lib.CameraGrads(_ptr(d_view), _ptr(d_proj), _ptr(d_cam), _ptr(cscratch), cbytes)
+                    cam_grads = (d_view.view(rs.viewmatrix.shape), d_proj.view(rs.projmatrix.shape),
+                                 d_cam.view(rs.campos.shape))
+                if ctx.depth_grad:   # one entry point for every combination with the alpha and camera gradients
+                    ga = None if grad_alpha is None else _f32c(grad_alpha, device)
+                    gd = _f32c(grad_depth, device)
+                    _lib.check(lib.gsr_backward_depth(C.byref(s), C.byref(c), state.cap, _ptr(geom), geom.numel(),
+                                                      _ptr(binning), binning.numel(), _ptr(img), img.numel(),
+                                                      _ptr(radii), _ptr(grad_out_color), _ptr(ga), _ptr(gd),
+                                                      _ptr(scratch), sbytes, C.byref(gr),
+                                                      None if cam is None else C.byref(cam), st), "gsr_backward_depth")
+                elif ctx.camera_grad:
                     ga = None if grad_alpha is None else _f32c(grad_alpha, device)
                     _lib.check(lib.gsr_backward_camera(C.byref(s), C.byref(c), state.cap, _ptr(geom), geom.numel(),
                                                        _ptr(binning), binning.numel(), _ptr(img), img.numel(),
                                                        _ptr(radii), _ptr(grad_out_color), _ptr(ga), _ptr(scratch), sbytes,
                                                        C.byref(gr), C.byref(cam), st), "gsr_backward_camera")
-                    cam_grads = (d_view.view(rs.viewmatrix.shape), d_proj.view(rs.projmatrix.shape),
-                                 d_cam.view(rs.campos.shape))
                 elif grad_alpha is not None:
                     grad_alpha = _f32c(grad_alpha, device)
                     _lib.check(lib.gsr_backward_alpha(C.byref(s), C.byref(c), state.cap, _ptr(geom), geom.numel(),
@@ -298,7 +310,7 @@ class _RasterizeGaussians(torch.autograd.Function):
                     dL_dscales.zero_(); dL_drotations.zero_()
         # same slots as the reference (__init__.py:213-223); autograd drops grads of inputs that do not need one
         grads = (dL_dmeans3D, dL_dmeans2D, dL_dsh, dL_dcolors, dL_dopacity, dL_dscales, dL_drotations, dL_dcov3D,
-                 None, None)
+                 None, None, None)
         if ctx.camera_grad:
             if P == 0:
                 z = lambda t: torch.zeros_like(t, dtype=torch.float32)
@@ -313,11 +325,12 @@ class _RasterizeGaussiansRaw(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, means3D, means2D, opacity_logits, features_dc, features_rest, log_scales, raw_rotations,
-                raster_settings):
+                raster_settings, depth_grad=False):
         empty = torch.empty(0, dtype=torch.float32, device=means3D.device)
         color, depth, state, inputs = _forward_impl(means3D, features_dc, empty, opacity_logits, log_scales,
                                                     raw_rotations, empty, raster_settings, raw_rest=features_rest)
         ctx.raster_settings = raster_settings
+        ctx.depth_grad = bool(depth_grad)
         ctx.state = state
         (m3, dc, _, op, sc, ro, _, rest) = inputs
         ctx.save_for_backward(m3, dc, rest, op, sc, ro, state.radii, state.geom, state.binning, state.img)
@@ -346,32 +359,45 @@ class _RasterizeGaussiansRaw(torch.autograd.Function):
                 sbytes = lib.gsr_backward_scratch_bytes(P)
                 scratch = torch.empty(sbytes, dtype=torch.uint8, device=device)
                 st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
-                _lib.check(lib.gsr_backward_raw(C.byref(s), C.byref(rc), state.cap, _ptr(geom), geom.numel(),
-                                                _ptr(binning), binning.numel(), _ptr(img), img.numel(), _ptr(radii),
-                                                _ptr(grad_out_color), _ptr(scratch), sbytes, C.byref(gr), st),
-                           "gsr_backward_raw")
-        return d_m3, d_m2, d_op, d_dc, d_rest, d_sc, d_ro, None
+                if ctx.depth_grad:
+                    gd = _f32c(grad_depth, device)
+                    _lib.check(lib.gsr_backward_raw_depth(C.byref(s), C.byref(rc), state.cap, _ptr(geom), geom.numel(),
+                                                          _ptr(binning), binning.numel(), _ptr(img), img.numel(),
+                                                          _ptr(radii), _ptr(grad_out_color), _ptr(gd), _ptr(scratch),
+                                                          sbytes, C.byref(gr), st), "gsr_backward_raw_depth")
+                else:
+                    _lib.check(lib.gsr_backward_raw(C.byref(s), C.byref(rc), state.cap, _ptr(geom), geom.numel(),
+                                                    _ptr(binning), binning.numel(), _ptr(img), img.numel(), _ptr(radii),
+                                                    _ptr(grad_out_color), _ptr(scratch), sbytes, C.byref(gr), st),
+                               "gsr_backward_raw")
+        return d_m3, d_m2, d_op, d_dc, d_rest, d_sc, d_ro, None, None
 
 
 class GaussianRasterizer(nn.Module):
-    def __init__(self, raster_settings, return_alpha: bool = False, camera_grad: bool = False):
+    def __init__(self, raster_settings, return_alpha: bool = False, camera_grad: bool = False,
+                 depth_grad: bool = False):
         """``return_alpha=True`` (opt-in, not in the reference) appends a fourth output to ``forward``: the alpha image
         ``1 - final_T`` [1,H,W] (the reference keeps final_T as ``accum_alpha`` but never returns it); it is
         differentiable like the colour.
         ``camera_grad=True`` (opt-in, not in the reference): ``raster_settings.viewmatrix / projmatrix / campos`` become
         differentiable inputs -- their ``.grad`` is filled by the backward (gsr_backward_camera), each array treated as an
-        independent input exactly as the forward reads it."""
+        independent input exactly as the forward reads it.
+        ``depth_grad=True`` (opt-in, not in the reference): the depth image (third output) becomes differentiable -- a
+        loss on it reaches means3D, means2D, opacities, scales, rotations / cov3D_precomp (and the view matrix with
+        ``camera_grad``) through gsr_backward_depth. Without the flag the gradient of the depth image is ignored, as in the
+        reference: a loss on it trains nothing. Applies to ``forward`` and ``forward_raw``."""
         super().__init__()
         self.raster_settings = raster_settings
         self.return_alpha = bool(return_alpha)
         self.camera_grad = bool(camera_grad)
+        self.depth_grad = bool(depth_grad)
 
     def forward_raw(self, means3D, means2D, opacity_logits, features_dc, features_rest, log_scales, raw_rotations):
         """Opt-in fused-activation call (not part of the reference API): the arguments are the scene model's raw
         parameters (``_xyz, _opacity, _features_dc, _features_rest, _scaling, _rotation``); sigmoid / exp / normalize
         and the SH concatenation happen inside the preprocess kernels. Same return tuple as ``forward``."""
         return _RasterizeGaussiansRaw.apply(means3D, means2D, opacity_logits, features_dc, features_rest, log_scales,
-                                            raw_rotations, self.raster_settings)
+                                            raw_rotations, self.raster_settings, self.depth_grad)
 
     def markVisible(self, positions):
         # __init__.py:248-256 / rasterize_points.cu:159-175
@@ -415,7 +441,7 @@ class GaussianRasterizer(nn.Module):
             cov3D_precomp = empty
 
         return rasterize_gaussians(means3D, means2D, shs, colors_precomp, opacities, scales, rotations,
-                                   cov3D_precomp, raster_settings, self.return_alpha, self.camera_grad)
+                                   cov3D_precomp, raster_settings, self.return_alpha, self.camera_grad, self.depth_grad)
 
     def apply_weights(self, means3D, means2D, opacities, shs=None, weights=None, scales=None, rotations=None,
                       cov3Ds_precomp=None, cnt=None, image_weights=None):

@@ -177,6 +177,23 @@ GSR_API int gsr_backward_camera(const gsr_settings* s, const gsr_cloud* c, int32
                         const float* dL_dout_alpha /* may be NULL */, void* scratch, size_t scratch_bytes,
                         const gsr_grads* grads, const gsr_camera_grads* camera, void* stream);
 
+/* ---- depth gradients (opt-in; the reference's backward ignores the gradient of its depth output) -----------------
+ * The forward's depth image D = sum_i d_i*alpha_i*T_i (d_i = view-space z of Gaussian i, no background term) is blended
+ * exactly like a colour channel. gsr_backward_depth is gsr_backward_camera with the additional upstream gradient
+ * dL_dout_depth [H*W] (REQUIRED: NULL is GSR_ERR_INVALID; pass zeros for "none") and with dL_dout_alpha and camera both
+ * optional (NULL = no alpha gradient / no camera gradients), so it covers every combination of the three extras. It adds
+ *   dL/dalpha_i += T_i * (d_i - depth blended behind i) * dL/dD   (-> mean2D, conic, opacity, and so on down the chain)
+ *   dL/dmean3D_i += (sum over pixels of alpha_i*T_i*dL/dD) * (view[2], view[6], view[10])
+ * and, with camera gradients, dL/dview[2 + 4r] += that sum * mean_r, dL/dview[14] += that sum. d_i is the unclamped
+ * view depth, so no clamp applies; projmatrix and campos receive nothing from the depth image.
+ * gsr_backward_raw_depth is gsr_backward_raw with the same additional dL_dout_depth. */
+GSR_API int gsr_backward_depth(const gsr_settings* s, const gsr_cloud* c, int32_t num_rendered, const void* geometry,
+                       size_t geometry_bytes, const void* binning, size_t binning_bytes, const void* image,
+                       size_t image_bytes, const int32_t* radii, const float* dL_dout_color,
+                       const float* dL_dout_alpha /* may be NULL */, const float* dL_dout_depth /* [H*W] */,
+                       void* scratch, size_t scratch_bytes, const gsr_grads* grads,
+                       const gsr_camera_grads* camera /* may be NULL */, void* stream);
+
 /* ---- markVisible: present[i] = view-space z > 0.2 (auxiliary.h:139-164) ------------------------------- */
 GSR_API int gsr_mark_visible(int32_t P, const float* means3D, const float* viewmatrix, const float* projmatrix,
                      uint8_t* present, void* stream);
@@ -247,6 +264,12 @@ GSR_API int gsr_backward_raw(const gsr_settings* s, const gsr_raw_cloud* c, int3
                      size_t geometry_bytes, const void* binning, size_t binning_bytes, const void* image,
                      size_t image_bytes, const int32_t* radii, const float* dL_dout_color, void* scratch,
                      size_t scratch_bytes, const gsr_raw_grads* grads, void* stream);
+/* gsr_backward_raw plus the gradient of the depth image, dL_dout_depth [H*W] (required; see gsr_backward_depth) */
+GSR_API int gsr_backward_raw_depth(const gsr_settings* s, const gsr_raw_cloud* c, int32_t num_rendered,
+                           const void* geometry, size_t geometry_bytes, const void* binning, size_t binning_bytes,
+                           const void* image, size_t image_bytes, const int32_t* radii, const float* dL_dout_color,
+                           const float* dL_dout_depth, void* scratch, size_t scratch_bytes, const gsr_raw_grads* grads,
+                           void* stream);
 
 /* ---- Gaussian-sharded multi-GPU path (BASELINE config 4; SURVEY.md 8(e)) ----------------------------------
  * The reference has no multi-GPU rasterizer; these entry points split the single-GPU pipeline at the two places
